@@ -15,6 +15,11 @@ One JSON line on stdout (rank 0). Keys follow the driver's contract:
   cpu_baseline the CPU oracle ("forma CPU path, restated") on the host cores
 `--impl reference` times that CPU restatement as its own arm (the Rust crate
 cannot be built here: no cargo/rustc, see DESIGN.md).
+
+`--dump-outputs DIR` writes the frames of the headline workload's last timed step (CUDA arm:
+frame_device.npy from render_device, frame_host.npy from the host-buffer call; reference arm:
+frame_host.npy) with pixel_index.npy, so that two builds can be compared pixel for pixel: the
+scenes are seeded, so the same arguments give the same inputs.
 """
 from __future__ import annotations
 
@@ -216,6 +221,9 @@ def run_reference(args):
     if rank != 0:
         return
     leg = cpu_leg(args.workload, args.steps, args.warmup)
+    if args.dump_outputs:
+        w, h, _ = WORKLOADS[args.workload]
+        dump_outputs(args.dump_outputs, {"frame_host": leg["frame"]}, w, h)
     fps = leg["fps"]
     out = {
         "impl": "reference", "metric": "frames/sec", "value": fps, "unit": "frames/s", "n_gpus": args.gpus,
@@ -465,6 +473,9 @@ def bench_workload(env, args, name, steps, warmup, headline):
             a["launches"] += v["launches"]
     dev_ms, wall_ms = timed(frame_device, steps, device_acc)
     c1 = renderer.counters()
+    # The device-resident frame of the last timed step, for --dump-outputs (rank 0 holds the whole frame);
+    # kept on the device until the timing below is over.
+    device_frame = (whole if world > 1 else fb).clone() if headline and args.dump_outputs and rank == 0 else None
     gather_ms = sum(a.elapsed_time(b) for a, b in gather_events[-steps:]) / steps if gather_events else 0.0
     render_ms = stage_acc["total"] / steps
     for _ in range(max(warmup, 1)):
@@ -576,7 +587,21 @@ def bench_workload(env, args, name, steps, warmup, headline):
     }
     out["_frame"] = frame_copy
     out["_frame_no"] = frame_no[0]
+    out["_device_frame"] = None if device_frame is None else device_frame.cpu().numpy().reshape(-1)
     return out
+
+
+def dump_outputs(path, frames, w, h, budget=1 << 20):
+    """Writes the RGBA8 frames (flat uint8, w * h * 4 bytes each) as float32 (n, 4) arrays of pixel
+    values in `path`/<name>.npy, with `pixel_index.npy` (float64, n): the row-major index y * w + x
+    of each of those n pixels. Frames of more than `budget` pixels are sampled at the same `budget`
+    pixels, drawn with a fixed seed, so that runs with the same arguments dump the same pixels."""
+    os.makedirs(path, exist_ok=True)
+    n = w * h
+    index = np.arange(n) if n <= budget else np.sort(np.random.default_rng(0).choice(n, budget, replace=False))
+    np.save(os.path.join(path, "pixel_index.npy"), index.astype(np.float64))
+    for name, frame in frames.items():
+        np.save(os.path.join(path, f"{name}.npy"), frame.reshape(n, 4)[index].astype(np.float32))
 
 
 def run_cuda(args):
@@ -617,7 +642,10 @@ def run_cuda(args):
         if world > 1:
             dist.destroy_process_group()
         return
-    frame, frame_no = res.pop("_frame"), res.pop("_frame_no")
+    frame, frame_no, device_frame = res.pop("_frame"), res.pop("_frame_no"), res.pop("_device_frame")
+    if args.dump_outputs:
+        w, h, _ = WORKLOADS[args.workload]
+        dump_outputs(args.dump_outputs, {"frame_device": device_frame, "frame_host": frame}, w, h)
     out = {"metric": "frames/sec", "value": res.pop("value"), "unit": res.pop("unit"), "n_gpus": world, "steps": args.steps,
            "warmup": args.warmup, "ms_per_step": res.pop("ms_per_step"), "higher_is_better": True, "scaling": "strong",
            "vs_baseline": None, "dtype": "f32+f64/u64", "data": data_of(args), "config": config_of(args, world)}
@@ -629,6 +657,7 @@ def run_cuda(args):
         for name, e in extras.items():
             e.pop("_frame")
             e.pop("_frame_no")
+            e.pop("_device_frame")
             e.pop("step_ms_trace", None)
             out["extra"][name] = e
     if world == 1 and not args.no_cpu:
@@ -673,7 +702,12 @@ def main():
                          "(default: circles8k_1m, BASELINE config 5, when the headline workload is paris4k)")
     ap.add_argument("--no-extra", action="store_true", help="headline workload only")
     ap.add_argument("--equal-bands", action="store_true", help="multi-GPU: equal tile-row bands instead of cost-balanced ones")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the frames of the headline workload's last timed step "
+                         "as DIR/<name>.npy (float32 pixel values; frames over 2^20 pixels as a fixed seeded sample of 2^20 pixels)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":

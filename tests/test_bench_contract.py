@@ -66,6 +66,54 @@ def test_reference_arm_under_torchrun_only_rank0_works():
     check_reference_line(lines[0], 2, 2)
 
 
+def oracle_smoke_frame():
+    import numpy as np
+
+    from forma_b200.binding import RGBA, Color
+    from oracle import oracle
+    from workloads import build_scene
+    api = oracle.load()
+    comp, w, h = build_scene(api, "smoke")
+    buf = np.zeros(w * h * 4, np.uint8)
+    api.Renderer().render(comp, buf, w, h, RGBA, Color(1.0, 1.0, 1.0, 0.0))
+    return buf.reshape(-1, 4).astype(np.float32)
+
+
+def check_dump(path, names):
+    import numpy as np
+    index = np.load(path / "pixel_index.npy")
+    assert index.dtype == np.float64 and np.array_equal(index, np.arange(640 * 360))
+    want = oracle_smoke_frame()
+    for name in names:
+        got = np.load(path / f"{name}.npy")
+        assert got.dtype == np.float32 and np.array_equal(got, want), name
+    assert sorted(p.name for p in path.iterdir()) == sorted(["pixel_index.npy"] + [f"{n}.npy" for n in names])
+
+
+def test_reference_arm_dumps_its_last_frame(tmp_path):
+    p = subprocess.run([sys.executable, BENCH, "--impl", "reference", "--workload", "smoke", "--steps", "2",
+                        "--dump-outputs", str(tmp_path / "out")], capture_output=True, text=True, timeout=300, cwd=ROOT)
+    assert p.returncode == 0, p.stderr[-2000:]
+    check_reference_line(json_lines(p.stdout)[0], 1, 2)
+    check_dump(tmp_path / "out", ["frame_host"])
+
+
+@pytest.mark.gpu
+def test_cuda_arm_dumps_the_frames_of_its_last_timed_step(tmp_path):
+    p = subprocess.run([sys.executable, BENCH, "--workload", "smoke", "--steps", "2", "--no-cpu",
+                        "--dump-outputs", str(tmp_path / "out")], capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert p.returncode == 0, p.stderr[-2000:]
+    d = json_lines(p.stdout)[0]
+    assert d["steps"] == 2 and len(d["step_ms_trace"]) == 2
+    check_dump(tmp_path / "out", ["frame_device", "frame_host"])
+
+
+def test_steps_below_one_are_refused():
+    p = subprocess.run([sys.executable, BENCH, "--impl", "reference", "--workload", "smoke", "--steps", "0"],
+                       capture_output=True, text=True, timeout=300, cwd=ROOT)
+    assert p.returncode != 0 and "--steps" in p.stderr and not json_lines(p.stdout)
+
+
 def test_cuda_arm_refuses_to_run_without_a_device():
     import torch
     if torch.cuda.is_available():

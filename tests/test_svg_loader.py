@@ -1,6 +1,7 @@
 """The SVG subset loader (forma_b200/svg.py, SURVEY.md §8(f) N1) against hand-computed
 expectations for every element it handles, against the committed paris-30k fixture, and
 through the CPU oracle for a picture-level check of arcs, rectangles and gradients."""
+import hashlib
 import math
 import os
 
@@ -131,14 +132,25 @@ def test_picture_through_the_oracle(parsed, oracle_api):
     assert xs.min() >= 39 and xs.max() <= 56 and ys.min() >= 23 and ys.max() <= 40
 
 
-def test_committed_fixture_matches_the_source_file():
-    src = "/root/reference/assets/svgs/paris-30k.svg"
-    if not os.path.exists(src):
-        pytest.skip("the reference checkout is not present (GPU box)")
-    fresh = svg.parse_svg(src)
+def test_committed_fixture_matches_the_source_file(tmp_path):
+    """The fixture is what the loader makes of paris-30k.svg. The source file (14 MB) is stood in
+    for by tests/golden/paris30k_excerpt.npz (tests/golden/make_paris_excerpt.py): digests of its
+    whole parse, and a seeded sample of its <path> elements, parsed afresh here."""
+    gold = np.load(os.path.join(ROOT, "tests", "golden", "paris30k_excerpt.npz"))
     fixture = svg.PathList.load(os.path.join(ROOT, "tests", "data", "paris30k_paths.npz"))
     for k in ("cmd", "pts", "cmd_off", "pt_off", "color", "fill_rule"):
-        assert np.array_equal(getattr(fresh, k), getattr(fixture, k)), k
+        a = getattr(fixture, k)
+        got = hashlib.sha256(a.dtype.str.encode() + str(a.shape).encode() + np.ascontiguousarray(a).tobytes()).hexdigest()
+        assert got == str(gold["sha256_" + k]), k
+    doc = tmp_path / "paris30k_excerpt.svg"
+    doc.write_bytes(gold["svg"].tobytes())
+    fresh = svg.parse_svg(str(doc))
+    index = gold["index"]
+    assert len(fresh) == len(index) > 300
+    for j, i in enumerate(index):
+        assert np.array_equal(fresh.cmd[fresh.cmd_off[j]:fresh.cmd_off[j + 1]], fixture.cmd[fixture.cmd_off[i]:fixture.cmd_off[i + 1]]), i
+        assert np.array_equal(fresh.pts[fresh.pt_off[j]:fresh.pt_off[j + 1]], fixture.pts[fixture.pt_off[i]:fixture.pt_off[i + 1]]), i
+        assert np.array_equal(fresh.color[j], fixture.color[i]) and fresh.fill_rule[j] == fixture.fill_rule[i], i
     assert len(fresh.weights) == 0 and not fresh.gradients
 
 
