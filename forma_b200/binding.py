@@ -74,6 +74,26 @@ BGR1 = (Channel.Blue, Channel.Green, Channel.Red, Channel.One)
 LAYER_LIMIT = (1 << 21) - 1
 
 
+class Format:
+    """Output format of a frame (FORMA_FORMAT_*): RGBA8 is sRGB bytes (cpu::Renderer);
+    RGBA16F / RGBA32F hold the painter's linear colour as is (gpu::Renderer's Rgba16Float
+    texture), 4 values per pixel."""
+
+    RGBA8, RGBA16F, RGBA32F = range(3)
+    BYTES_PER_PIXEL = {RGBA8: 4, RGBA16F: 8, RGBA32F: 16}
+    DTYPES = {RGBA8: np.uint8, RGBA16F: np.float16, RGBA32F: np.float32}
+    NAMES = {"rgba8": RGBA8, "rgba16f": RGBA16F, "rgba32f": RGBA32F}
+
+    @staticmethod
+    def of_dtype(dtype) -> int:
+        """uint8 -> RGBA8, float16 -> RGBA16F, float32 -> RGBA32F."""
+        dt = np.dtype(dtype)
+        for f, d in Format.DTYPES.items():
+            if dt == np.dtype(d):
+                return f
+        raise ValueError(f"no frame format stores {dt}: use uint8, float16 or float32")
+
+
 class OrderError(ValueError):
     pass
 
@@ -273,6 +293,8 @@ SIGNATURES = {
     "layer_cache_clear": (None, [_vp]),
     "renderer_render": (C.c_int, [_vp, _vp, _vp, C.c_uint64, C.c_uint64, C.c_uint64, _u32p, _fp, C.POINTER(_CRect), _vp, C.POINTER(_CTimings)]),
     "renderer_render_device": (C.c_int, [_vp, _vp, _vp, C.c_uint64, C.c_uint64, C.c_uint64, _u32p, _fp, C.POINTER(_CRect), _vp, C.POINTER(_CTimings)]),
+    "renderer_render_format": (C.c_int, [_vp, _vp, _vp, C.c_uint32, C.c_uint64, C.c_uint64, C.c_uint64, _u32p, _fp, C.POINTER(_CRect), _vp, C.POINTER(_CTimings)]),
+    "renderer_render_device_format": (C.c_int, [_vp, _vp, _vp, C.c_uint32, C.c_uint64, C.c_uint64, C.c_uint64, _u32p, _fp, C.POINTER(_CRect), _vp, C.POINTER(_CTimings)]),
     "renderer_launch_count": (C.c_uint64, [_vp]),
     "renderer_stage_times": (None, [_vp, C.POINTER(C.c_double)]),
     "renderer_counters": (None, [_vp, _u64p]),
@@ -295,11 +317,19 @@ SIGNATURES = {
     "renderer_multi_device_count": (C.c_int, [_vp]),
     "renderer_multi_render": (C.c_int, [_vp, _vp, _vp, C.c_uint64, C.c_uint64, C.c_uint64, _u32p, _fp, C.POINTER(_CRect), C.POINTER(_CTimings)]),
     "renderer_multi_render_device": (C.c_int, [_vp, _vp, _vp, C.c_uint64, C.c_uint64, C.c_uint64, _u32p, _fp, C.POINTER(_CRect), C.POINTER(_CTimings)]),
+    "renderer_multi_render_format": (C.c_int, [_vp, _vp, _vp, C.c_uint32, C.c_uint64, C.c_uint64, C.c_uint64, _u32p, _fp, C.POINTER(_CRect), C.POINTER(_CTimings)]),
+    "renderer_multi_render_device_format": (C.c_int, [_vp, _vp, _vp, C.c_uint32, C.c_uint64, C.c_uint64, C.c_uint64, _u32p, _fp, C.POINTER(_CRect), C.POINTER(_CTimings)]),
     "renderer_multi_bands": (C.c_int, [_vp, _u32p, C.POINTER(C.c_double)]),
     "renderer_row_costs": (C.c_uint64, [_vp, C.c_uint64, _u64p]),
     "set_option": (C.c_int, [C.c_char_p, C.c_int]),
     "get_option": (C.c_int, [C.c_char_p, C.POINTER(C.c_int)]),
 }
+
+
+# The float-frame entry points: a library that renders RGBA8 frames only may lack them (its
+# Renderer.render / render_device then refuse float buffers with FormaError).
+FORMAT_SYMBOLS = ("renderer_render_format", "renderer_render_device_format", "renderer_multi_render_format",
+                  "renderer_multi_render_device_format")
 
 
 class Api:
@@ -311,11 +341,18 @@ class Api:
             try:
                 fn = getattr(lib, prefix + name)
             except AttributeError:
-                if name in optional:
+                if name in optional or name in FORMAT_SYMBOLS:
                     continue
                 raise
             fn.restype, fn.argtypes = res, args
             setattr(self, name + "_fn" if name in ("set_option", "get_option") else name, fn)
+
+    def format_call(self, name: str, what: str):
+        """The float-frame entry point `name`, or FormaError when this library has none."""
+        fn = getattr(self, name, None)
+        if fn is None:
+            raise FormaError(f"{what}: this library renders RGBA8 frames only (no {self.prefix}{name})")
+        return fn
 
     def check(self, status: int, what: str) -> None:
         if status == 0:
@@ -633,7 +670,7 @@ class Renderer:
     (composition, buffer(width, stride, height), channels, clear_color, crop)."""
 
     def __init__(self, api: Api, device: int = 0):
-        self._api = api
+        self._api, self.device = api, device
         self._h = api.renderer_new(device)
         if not self._h:
             msg = api.last_error().decode() if hasattr(api, "last_error") else ""
@@ -654,33 +691,70 @@ class Renderer:
     def render(self, composition: Composition, buffer: np.ndarray, width: int, height: int,
                channels=RGBA, clear_color: Color = Color(1.0, 1.0, 1.0, 1.0), crop: Optional[Rect] = None,
                layer_cache: Optional[LayerCache] = None, stride: Optional[int] = None, timings: bool = True) -> Optional[Timings]:
-        """`buffer`: writable contiguous uint8 host array of >= height*stride bytes.
+        """`buffer`: writable contiguous host array of >= height*stride bytes. Its dtype picks the
+        frame format (Format.of_dtype): uint8 -> RGBA8 (sRGB bytes), float16 -> RGBA16F,
+        float32 -> RGBA32F (linear values), 4 values per pixel; `stride` is in bytes
+        (default width * bytes per pixel).
         timings=False passes a null `forma_timings*`: the call then does not query its stage events
         (stage_times() still can, afterwards)."""
-        stride = width * 4 if stride is None else stride
-        assert buffer.dtype == np.uint8 and buffer.flags["C_CONTIGUOUS"] and buffer.size >= height * stride
+        fmt = Format.of_dtype(buffer.dtype)
+        stride = width * Format.BYTES_PER_PIXEL[fmt] if stride is None else stride
+        assert buffer.flags["C_CONTIGUOUS"] and buffer.nbytes >= height * stride
         ch, cc, rect = self._common(channels, clear_color, crop)
         t = _CTimings() if timings else None
-        st = self._api.renderer_render(
-            self._h, composition._h, buffer.ctypes.data_as(C.c_void_p), width, stride, height, ch, cc,
-            C.byref(rect) if rect is not None else None, layer_cache._h if layer_cache else None,
-            C.byref(t) if t is not None else None)
+        args = (width, stride, height, ch, cc, C.byref(rect) if rect is not None else None,
+                layer_cache._h if layer_cache else None, C.byref(t) if t is not None else None)
+        if fmt == Format.RGBA8:
+            st = self._api.renderer_render(self._h, composition._h, buffer.ctypes.data_as(C.c_void_p), *args)
+        else:
+            st = self._api.format_call("renderer_render_format", "Renderer::render")(self._h, composition._h, buffer.ctypes.data_as(C.c_void_p), fmt, *args)
         self._api.check(st, "Renderer::render")
         return Timings(t.line_setup_ms, t.rasterize_ms, t.sort_ms, t.paint_ms, t.n_lines, t.n_segments) if t is not None else None
 
     def render_device(self, composition: Composition, device_ptr: int, width: int, height: int,
                       channels=RGBA, clear_color: Color = Color(1.0, 1.0, 1.0, 1.0), crop: Optional[Rect] = None,
                       layer_cache: Optional[LayerCache] = None, stride: Optional[int] = None,
-                      timings: bool = True) -> Optional[Timings]:
-        stride = width * 4 if stride is None else stride
+                      timings: bool = True, format: int = Format.RGBA8) -> Optional[Timings]:
+        """The frame stays in device memory at `device_ptr`, in `format` (a Format constant);
+        `stride` in bytes, default width * bytes per pixel."""
+        if format not in Format.BYTES_PER_PIXEL:
+            raise FormaError(f"Renderer::render_device: unknown format {format}")
+        stride = width * Format.BYTES_PER_PIXEL[format] if stride is None else stride
         ch, cc, rect = self._common(channels, clear_color, crop)
         t = _CTimings() if timings else None
-        st = self._api.renderer_render_device(
-            self._h, composition._h, C.c_void_p(device_ptr), width, stride, height, ch, cc,
-            C.byref(rect) if rect is not None else None, layer_cache._h if layer_cache else None,
-            C.byref(t) if t is not None else None)
+        args = (width, stride, height, ch, cc, C.byref(rect) if rect is not None else None,
+                layer_cache._h if layer_cache else None, C.byref(t) if t is not None else None)
+        if format == Format.RGBA8:
+            st = self._api.renderer_render_device(self._h, composition._h, C.c_void_p(device_ptr), *args)
+        else:
+            st = self._api.format_call("renderer_render_device_format", "Renderer::render_device")(self._h, composition._h, C.c_void_p(device_ptr), format, *args)
         self._api.check(st, "Renderer::render_device")
         return Timings(t.line_setup_ms, t.rasterize_ms, t.sort_ms, t.paint_ms, t.n_lines, t.n_segments) if t is not None else None
+
+    def render_tensor(self, composition: Composition, out, channels=RGBA, clear_color: Color = Color(1.0, 1.0, 1.0, 1.0),
+                      crop: Optional[Rect] = None, layer_cache: Optional[LayerCache] = None,
+                      timings: bool = True) -> Optional[Timings]:
+        """Renders into the CUDA tensor `out` of shape [H, W, 4] on this renderer's device: dtype
+        uint8 (RGBA8), float16 (RGBA16F) or float32 (RGBA32F). Its last two dims must be
+        contiguous; the row stride is out.stride(0).
+        The frame is rendered on torch.cuda.current_stream(device): this sets the renderer's
+        stream to it (set_stream), so later calls on this renderer run on that stream too, and
+        the tensor is ready for work queued on it afterwards without a synchronisation."""
+        import torch  # only this method needs torch
+
+        if not isinstance(out, torch.Tensor) or not out.is_cuda or out.device.index != self.device:
+            raise FormaError(f"Renderer::render_tensor: `out` must be a CUDA tensor on cuda:{self.device}")
+        dtypes = {torch.uint8: Format.RGBA8, torch.float16: Format.RGBA16F, torch.float32: Format.RGBA32F}
+        if out.dtype not in dtypes:
+            raise FormaError(f"Renderer::render_tensor: dtype {out.dtype} is not uint8, float16 or float32")
+        if out.dim() != 3 or out.shape[2] != 4 or out.shape[0] < 1 or out.shape[1] < 1:
+            raise FormaError(f"Renderer::render_tensor: shape {tuple(out.shape)} is not [H, W, 4]")
+        if out.stride(2) != 1 or out.stride(1) != 4 or out.stride(0) < 4 * out.shape[1]:
+            raise FormaError(f"Renderer::render_tensor: strides {out.stride()} (the last two dims must be contiguous)")
+        h, w = int(out.shape[0]), int(out.shape[1])
+        self.set_stream(torch.cuda.current_stream(out.device).cuda_stream)
+        return self.render_device(composition, out.data_ptr(), w, h, channels, clear_color, crop, layer_cache,
+                                  out.stride(0) * out.element_size(), timings, dtypes[out.dtype])
 
     def launch_count(self) -> int:
         return int(self._api.renderer_launch_count(self._h))
@@ -780,28 +854,37 @@ class MultiRenderer:
             raise FormaError(f"MultiRenderer::new failed: {api.last_error().decode()}")
         self.n = int(api.renderer_multi_device_count(self._h))
 
-    def _call(self, fn, what, composition, ptr, width, height, channels, clear_color, crop, stride):
-        stride = width * 4 if stride is None else stride
+    def _call(self, fn, what, composition, ptr, width, height, channels, clear_color, crop, stride, fmt=Format.RGBA8):
+        stride = width * Format.BYTES_PER_PIXEL[fmt] if stride is None else stride
         ch = (C.c_uint32 * 4)(*channels)
         cc = (C.c_float * 4)(clear_color.r, clear_color.g, clear_color.b, clear_color.a)
         rect = _CRect(crop.horizontal[0], crop.horizontal[1], crop.vertical[0], crop.vertical[1]) if crop is not None else None
         t = _CTimings()
-        st = fn(self._h, composition._h, ptr, width, stride, height, ch, cc, C.byref(rect) if rect is not None else None, C.byref(t))
+        head = (self._h, composition._h, ptr) + ((fmt,) if fmt != Format.RGBA8 else ())
+        st = fn(*head, width, stride, height, ch, cc, C.byref(rect) if rect is not None else None, C.byref(t))
         self._api.check(st, what)
         return Timings(t.line_setup_ms, t.rasterize_ms, t.sort_ms, t.paint_ms, t.n_lines, t.n_segments)
 
     def render(self, composition: "Composition", buffer: np.ndarray, width: int, height: int, channels=RGBA,
                clear_color: Color = Color(1.0, 1.0, 1.0, 1.0), crop: Optional[Rect] = None, stride: Optional[int] = None) -> Timings:
-        s = width * 4 if stride is None else stride
-        assert buffer.dtype == np.uint8 and buffer.flags["C_CONTIGUOUS"] and buffer.size >= height * s
-        return self._call(self._api.renderer_multi_render, "MultiRenderer::render", composition,
-                          buffer.ctypes.data_as(C.c_void_p), width, height, channels, clear_color, crop, stride)
+        """The buffer's dtype picks the format as in Renderer.render."""
+        fmt = Format.of_dtype(buffer.dtype)
+        s = width * Format.BYTES_PER_PIXEL[fmt] if stride is None else stride
+        assert buffer.flags["C_CONTIGUOUS"] and buffer.nbytes >= height * s
+        fn = (self._api.renderer_multi_render if fmt == Format.RGBA8
+              else self._api.format_call("renderer_multi_render_format", "MultiRenderer::render"))
+        return self._call(fn, "MultiRenderer::render", composition, buffer.ctypes.data_as(C.c_void_p), width, height, channels,
+                          clear_color, crop, stride, fmt)
 
     def render_device(self, composition: "Composition", device_ptr: int, width: int, height: int, channels=RGBA,
                       clear_color: Color = Color(1.0, 1.0, 1.0, 1.0), crop: Optional[Rect] = None,
-                      stride: Optional[int] = None) -> Timings:
-        return self._call(self._api.renderer_multi_render_device, "MultiRenderer::render_device", composition,
-                          C.c_void_p(device_ptr), width, height, channels, clear_color, crop, stride)
+                      stride: Optional[int] = None, format: int = Format.RGBA8) -> Timings:
+        if format not in Format.BYTES_PER_PIXEL:
+            raise FormaError(f"MultiRenderer::render_device: unknown format {format}")
+        fn = (self._api.renderer_multi_render_device if format == Format.RGBA8
+              else self._api.format_call("renderer_multi_render_device_format", "MultiRenderer::render_device"))
+        return self._call(fn, "MultiRenderer::render_device", composition, C.c_void_p(device_ptr), width, height, channels,
+                          clear_color, crop, stride, format)
 
     def bands(self):
         """(tile-row boundaries of the next frame's bands, ms of every band in the last frame)."""

@@ -138,6 +138,23 @@ struct PaintScene {
     uint32_t clear_unchanged;     // previous clear colour == this frame's
 };
 
+// Output buffer of a frame: format and, for float formats with a layer cache, the per-tile solid
+// colour at output precision (4 x f32 bits, or 4 x f16 in .x / .y; PaintScene::cache_tiles[].y is
+// unused then). Kept out of PaintScene so that the RGBA8 paint kernel's parameters stay as they were.
+struct FrameOut {
+    uint32_t format = 0;                // kFormat*
+    uint4* cache_solid_wide = nullptr;  // null without a cache and for RGBA8
+};
+
+// Output formats of the frame buffer (= FORMA_FORMAT_* in include/forma_b200.h).
+constexpr uint32_t kFormatRgba8 = 0, kFormatRgba16f = 1, kFormatRgba32f = 2;
+__host__ __device__ constexpr uint32_t format_bytes_per_pixel(uint32_t f) {
+    return f == kFormatRgba32f ? 16u : (f == kFormatRgba16f ? 8u : 4u);
+}
+__host__ __device__ constexpr uint32_t format_element_bytes(uint32_t f) {
+    return f == kFormatRgba32f ? 4u : (f == kFormatRgba16f ? 2u : 1u);
+}
+
 uint32_t cell_num_blocks(uint32_t n);
 // Cells in one pass over the sorted segments (+ a small kernel for the cells that cross a
 // CTA tile): cell_start[c] = first segment of cell c (cell_start[#cells] = n), the cell's
@@ -194,7 +211,8 @@ constexpr int kHeavyListClasses = 4;
 void launch_tile_index(const PaintScene& S, const uint64_t* ekey, uint32_t n_entries, uint2* tile_range, uint32_t* heavy,
                        uint32_t* heavy_count, cudaStream_t st, const DevCounts& dc = DevCounts());
 void launch_paint(const PaintScene& S, const uint64_t* segs, const EntryRec* recs, const uint2* tile_range, const uint32_t* heavy,
-                  const uint32_t* heavy_count, uint8_t* eflags, uint8_t* framebuffer, uint32_t* tile_counter, cudaStream_t st);
+                  const uint32_t* heavy_count, uint8_t* eflags, uint8_t* framebuffer, uint32_t* tile_counter, cudaStream_t st,
+                  const FrameOut& out = FrameOut());
 // GradRec of every style slot (see device_types.h).
 void launch_grad_setup(const StyleRec* styles, const StopRec* stops, uint32_t n_styles, GradRec* grads, cudaStream_t st);
 // Packed fp32 (f32x2) arithmetic of the painter against scalar IEEE operations; mismatches are added to out[0].
@@ -202,7 +220,7 @@ void launch_f32x2_selftest(const float* a, const float* b, const float* c, uint3
 // out[row] = 32 x entries + pixel segments of tile row `row` (see row_cost_kernel).
 void launch_row_costs(const uint2* tile_range, uint32_t tiles_x, uint32_t tiles_y, const uint64_t* segs, uint32_t n,
                       unsigned long long* out, cudaStream_t st, unsigned long long* seg_out = nullptr);
-// Packs the tiles in S.written_list into `packed` (256 u32 per tile, row-major).
-void launch_gather_tiles(const PaintScene& S, const uint8_t* framebuffer, uint32_t* packed, cudaStream_t st);
+// Packs the tiles in S.written_list into `packed` (256 pixels of `format` per tile, row-major).
+void launch_gather_tiles(const PaintScene& S, uint32_t format, const uint8_t* framebuffer, void* packed, cudaStream_t st);
 
 }  // namespace forma

@@ -32,6 +32,11 @@
 // (tile_index_kernel sorts them into four classes by entry count): a tile is painted by
 // one warp from its first to its last layer, so the heaviest tile bounds the kernel's
 // tail unless it starts early (longest-processing-time order).
+//
+// The output format is a template parameter of the kernel: RGBA8 encodes to sRGB bytes
+// (compute_srgb), RGBA16F / RGBA32F store the same four linear values compute_srgb would
+// receive, in channel order, as IEEE binary16 (round to nearest even) or binary32.
+#include <cuda_fp16.h>
 #include <mutex>
 #include "paint_common.cuh"
 #include "paint_math.cuh"
@@ -48,6 +53,7 @@ struct PaintInputs {
     uint8_t* eflags;             // per sorted entry: optimizer flags, initialised with EntryRec::flags0
     uint8_t* framebuffer;
     uint32_t* tile_counter;
+    uint4* cache_solid_wide;     // FrameOut::cache_solid_wide (float formats)
 };
 
 __device__ __forceinline__ uint32_t meta_fill_rule(uint32_t m) { return m & 1u; }
@@ -203,6 +209,65 @@ __device__ __forceinline__ void store_tile_solid(const PaintScene& S, uint8_t* f
         for (int j = 0; j < 8; ++j)
             if (px0 + (uint32_t)j < S.width) reinterpret_cast<uint32_t*>(row)[j] = rgba;
     }
+}
+
+// ---------------------------------------------------------------------------
+// Float frames. A pixel is 16 B (RGBA32F: four f32) or 8 B (RGBA16F: four f16,
+// __floats2half2_rn); its "wide" form is a uint4 holding those bytes (f16: in .x / .y).
+// ---------------------------------------------------------------------------
+__device__ __forceinline__ float4 select_channels(float r, float g, float b, float a, const uint32_t* ch) {
+    const Rgba c{r, g, b, a};
+    return make_float4(channel_of(c, ch[0]), channel_of(c, ch[1]), channel_of(c, ch[2]), channel_of(c, ch[3]));
+}
+__device__ __forceinline__ uint32_t half2_bits(float lo, float hi) {
+    const __half2 h = __floats2half2_rn(lo, hi);  // .x (low 16 bits, first in memory) = lo
+    return *reinterpret_cast<const uint32_t*>(&h);
+}
+template <uint32_t kFormat>
+__device__ __forceinline__ uint4 wide_of(float4 v) {
+    if (kFormat == kFormatRgba32f) return make_uint4(__float_as_uint(v.x), __float_as_uint(v.y), __float_as_uint(v.z), __float_as_uint(v.w));
+    return make_uint4(half2_bits(v.x, v.y), half2_bits(v.z, v.w), 0u, 0u);
+}
+// One pixel at an address aligned to the element size only.
+template <uint32_t kFormat>
+__device__ __forceinline__ void store_pixel_scalar(uint8_t* p, uint4 w) {
+    if (kFormat == kFormatRgba32f) {
+        uint32_t* d = reinterpret_cast<uint32_t*>(p);
+        d[0] = w.x; d[1] = w.y; d[2] = w.z; d[3] = w.w;
+    } else {
+        uint16_t* d = reinterpret_cast<uint16_t*>(p);
+        d[0] = (uint16_t)w.x; d[1] = (uint16_t)(w.x >> 16); d[2] = (uint16_t)w.y; d[3] = (uint16_t)(w.y >> 16);
+    }
+}
+// Pixels x, x + 1 of a lane's run (x even; p = their address). `vec`: the run is whole and
+// 16-byte aligned: 16-byte stores (RGBA32F one per pixel, RGBA16F one per pair).
+template <uint32_t kFormat>
+__device__ __forceinline__ void store_pair(uint8_t* p, uint4 w0, uint4 w1, bool vec, uint32_t x, uint32_t width) {
+    constexpr uint32_t kBpp = format_bytes_per_pixel(kFormat);
+    if (vec) {
+        if (kFormat == kFormatRgba32f) {
+            reinterpret_cast<uint4*>(p)[0] = w0;
+            reinterpret_cast<uint4*>(p)[1] = w1;
+        } else {
+            reinterpret_cast<uint4*>(p)[0] = make_uint4(w0.x, w0.y, w1.x, w1.y);
+        }
+    } else {
+        if (x < width) store_pixel_scalar<kFormat>(p, w0);
+        if (x + 1u < width) store_pixel_scalar<kFormat>(p + kBpp, w1);
+    }
+}
+
+template <uint32_t kFormat>
+__device__ __forceinline__ void store_tile_solid_wide(const PaintScene& S, uint8_t* fb, uint32_t tx, uint32_t ty, uint32_t lane,
+                                                      uint4 w, bool vec_ok) {
+    constexpr uint32_t kBpp = format_bytes_per_pixel(kFormat);
+    const uint32_t py = ty * 16u + (lane >> 1);
+    const uint32_t px0 = tx * 16u + (lane & 1u) * 8u;
+    if (py >= S.height || px0 >= S.width) return;
+    uint8_t* row = fb + (size_t)py * S.stride + (size_t)px0 * kBpp;
+    const bool vec = vec_ok && px0 + 8u <= S.width;
+#pragma unroll
+    for (uint32_t j = 0; j < 8u; j += 2u) store_pair<kFormat>(row + j * kBpp, w, w, vec, px0 + j, S.width);
 }
 
 // Shared-memory word of pixel (local_x, local_y): row-major, ly * 16 + lx, i.e. the segment's
@@ -380,7 +445,7 @@ __device__ __forceinline__ void scatter_entry(const uint64_t* __restrict__ segs,
     if (n > 64u) scatter_rest(segs, s0 + 64u, s1, cells, lane);
 }
 
-template <int kMinBlocks>
+template <int kMinBlocks, uint32_t kFormat>
 __global__ void __launch_bounds__(kPaintWarpsPerBlock * 32, kMinBlocks) paint_kernel(PaintScene S, PaintInputs in, uint32_t n_tiles) {
     __shared__ __align__(16) WarpSmem s_warp[kPaintWarpsPerBlock];
     const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31u;
@@ -598,14 +663,33 @@ __global__ void __launch_bounds__(kPaintWarpsPerBlock * 32, kMinBlocks) paint_ke
                 }
             }
             if (solid) {
-                const uint32_t bytes = solid_to_srgb_bytes(dst, S.channels);
-                // CachedTile::convert_optimizer_op (cpu/painter/mod.rs:686-704): the same
-                // solid colour as last frame is not written again.
-                const bool same = use_cache && ((cache_x >> 30) & 1u) && cache_solid == bytes;
-                if (!same) store_tile_solid(S, in.framebuffer, tx, ty, lane, bytes, vec_ok);
-                if (lane == 0) {
-                    if (use_cache) S.cache_tiles[tid] = make_uint2(cache_x | (1u << 30), bytes);
-                    if (!same && S.written_list) S.written_list[atomicAdd(S.written_count, 1u)] = tid;
+                if constexpr (kFormat == kFormatRgba8) {
+                    const uint32_t bytes = solid_to_srgb_bytes(dst, S.channels);
+                    // CachedTile::convert_optimizer_op (cpu/painter/mod.rs:686-704): the same
+                    // solid colour as last frame is not written again.
+                    const bool same = use_cache && ((cache_x >> 30) & 1u) && cache_solid == bytes;
+                    if (!same) store_tile_solid(S, in.framebuffer, tx, ty, lane, bytes, vec_ok);
+                    if (lane == 0) {
+                        if (use_cache) S.cache_tiles[tid] = make_uint2(cache_x | (1u << 30), bytes);
+                        if (!same && S.written_list) S.written_list[atomicAdd(S.written_count, 1u)] = tid;
+                    }
+                } else {
+                    // The same rule at the output precision: the colour is compared as the
+                    // f16 / f32 bits the frame holds (side array in.cache_solid_wide).
+                    const uint4 w = wide_of<kFormat>(select_channels(dst.r, dst.g, dst.b, dst.a, S.channels));
+                    bool same = false;
+                    if (use_cache && ((cache_x >> 30) & 1u)) {
+                        const uint4 c = in.cache_solid_wide[tid];
+                        same = c.x == w.x && c.y == w.y && c.z == w.z && c.w == w.w;
+                    }
+                    if (!same) store_tile_solid_wide<kFormat>(S, in.framebuffer, tx, ty, lane, w, vec_ok);
+                    if (lane == 0) {
+                        if (use_cache) {
+                            S.cache_tiles[tid] = make_uint2(cache_x | (1u << 30), cache_solid);
+                            in.cache_solid_wide[tid] = w;
+                        }
+                        if (!same && S.written_list) S.written_list[atomicAdd(S.written_count, 1u)] = tid;
+                    }
                 }
                 continue;
             }
@@ -854,7 +938,27 @@ __global__ void __launch_bounds__(kPaintWarpsPerBlock * 32, kMinBlocks) paint_ke
 
         // compute_srgb + LinearLayout::write (mod.rs:466-483, layout/mod.rs:265-282).
         const uint32_t py = ty * 16u + row;
-        if (py < S.height && x0 < S.width) {
+        if constexpr (kFormat != kFormatRgba8) {
+            // Float frames: the accumulator as is, channel-selected, no encode.
+            if (py < S.height && x0 < S.width) {
+                constexpr uint32_t kBpp = format_bytes_per_pixel(kFormat);
+                uint8_t* rowp = in.framebuffer + (size_t)py * S.stride + (size_t)x0 * kBpp;
+                const bool vec = vec_ok && x0 + 8u <= S.width;
+#pragma unroll
+                for (int q = 0; q < 4; ++q) {
+                    float4 p0, p1;
+                    if (rgba_order) {
+                        p0 = make_float4(dr[q].x, dg[q].x, db[q].x, da[q].x);
+                        p1 = make_float4(dr[q].y, dg[q].y, db[q].y, da[q].y);
+                    } else {
+                        p0 = select_channels(dr[q].x, dg[q].x, db[q].x, da[q].x, S.channels);
+                        p1 = select_channels(dr[q].y, dg[q].y, db[q].y, da[q].y, S.channels);
+                    }
+                    store_pair<kFormat>(rowp + 2u * (uint32_t)q * kBpp, wide_of<kFormat>(p0), wide_of<kFormat>(p1), vec,
+                                        x0 + 2u * (uint32_t)q, S.width);
+                }
+            }
+        } else if (py < S.height && x0 < S.width) {
             uint32_t out[8];
             if (rgba_order) {
 #pragma unroll
@@ -887,32 +991,44 @@ __global__ void __launch_bounds__(kPaintWarpsPerBlock * 32, kMinBlocks) paint_ke
     }
 }
 
-// Packs the tiles named in `list` (written by paint_kernel) into 1 KB records,
-// row-major 16x16 RGBA8, so that a damaged frame costs a device->host copy
-// proportional to the damage. One warp per tile.
+// Packs the tiles named in `list` (written by paint_kernel) into records of 256 pixels,
+// row-major 16x16 (1 KB for RGBA8), so that a damaged frame costs a device->host copy
+// proportional to the damage. One warp per tile. A pixel is kPerPixel elements of type E,
+// each read at its own address: a float frame's stride need only be a multiple of E.
+template <typename E, int kPerPixel>
 __global__ void __launch_bounds__(256) gather_tiles_kernel(const uint8_t* __restrict__ fb, uint32_t stride, uint32_t width,
                                                            uint32_t height, uint32_t tiles_x,
                                                            const uint32_t* __restrict__ list,
-                                                           const uint32_t* __restrict__ count, uint32_t* __restrict__ out) {
+                                                           const uint32_t* __restrict__ count, E* __restrict__ out) {
     const uint32_t n = *count;
     const uint32_t lane = threadIdx.x & 31u;
     for (uint32_t i = blockIdx.x * 8u + (threadIdx.x >> 5); i < n; i += gridDim.x * 8u) {
         const uint32_t tid = list[i];
         const uint32_t x0 = (tid % tiles_x) * 16u, y0 = (tid / tiles_x) * 16u;
 #pragma unroll
-        for (int k = 0; k < 8; ++k) {
-            const uint32_t p = (uint32_t)k * 32u + lane;  // pixel index in the tile, row-major
-            const uint32_t x = x0 + (p & 15u), y = y0 + (p >> 4);
-            uint32_t v = 0;
-            if (x < width && y < height) v = *reinterpret_cast<const uint32_t*>(fb + (size_t)y * stride + (size_t)x * 4u);
-            out[(size_t)i * 256u + p] = v;
+        for (int k = 0; k < 8 * kPerPixel; ++k) {
+            const uint32_t p = (uint32_t)k * 32u + lane;  // element index in the tile record
+            const uint32_t px = p / (uint32_t)kPerPixel, e = p % (uint32_t)kPerPixel;  // pixel index in the tile, row-major
+            const uint32_t x = x0 + (px & 15u), y = y0 + (px >> 4);
+            E v = 0;
+            if (x < width && y < height)
+                v = *reinterpret_cast<const E*>(fb + (size_t)y * stride + ((size_t)x * kPerPixel + e) * sizeof(E));
+            out[(size_t)i * (256u * kPerPixel) + p] = v;
         }
     }
 }
 
-void launch_gather_tiles(const PaintScene& S, const uint8_t* framebuffer, uint32_t* packed, cudaStream_t st) {
-    gather_tiles_kernel<<<device_sm_count() * 4, 256, 0, st>>>(framebuffer, S.stride, S.width, S.height, S.tiles_x, S.written_list,
-                                                               S.written_count, packed);
+void launch_gather_tiles(const PaintScene& S, uint32_t format, const uint8_t* framebuffer, void* packed, cudaStream_t st) {
+    const int grid = device_sm_count() * 4;
+    if (format == kFormatRgba32f)
+        gather_tiles_kernel<uint32_t, 4><<<grid, 256, 0, st>>>(framebuffer, S.stride, S.width, S.height, S.tiles_x, S.written_list,
+                                                               S.written_count, static_cast<uint32_t*>(packed));
+    else if (format == kFormatRgba16f)
+        gather_tiles_kernel<uint16_t, 4><<<grid, 256, 0, st>>>(framebuffer, S.stride, S.width, S.height, S.tiles_x, S.written_list,
+                                                               S.written_count, static_cast<uint16_t*>(packed));
+    else
+        gather_tiles_kernel<uint32_t, 1><<<grid, 256, 0, st>>>(framebuffer, S.stride, S.width, S.height, S.tiles_x, S.written_list,
+                                                               S.written_count, static_cast<uint32_t*>(packed));
 }
 
 // One thread per style slot: the GradRec of a gradient of up to four stops, with the very
@@ -988,31 +1104,37 @@ void launch_f32x2_selftest(const float* a, const float* b, const float* c, uint3
 }
 
 void launch_paint(const PaintScene& S, const uint64_t* segs, const EntryRec* recs, const uint2* tile_range, const uint32_t* heavy,
-                  const uint32_t* heavy_count, uint8_t* eflags, uint8_t* framebuffer, uint32_t* tile_counter, cudaStream_t st) {
+                  const uint32_t* heavy_count, uint8_t* eflags, uint8_t* framebuffer, uint32_t* tile_counter, cudaStream_t st,
+                  const FrameOut& out) {
     if (S.tx_hi <= S.tx_lo || S.ty_hi <= S.ty_lo) return;
     uint32_t n_tiles = (S.tx_hi - S.tx_lo) * (S.ty_hi - S.ty_lo);
     cudaMemsetAsync(tile_counter, 0, sizeof(uint32_t), st);
-    PaintInputs in{segs, recs, tile_range, heavy, heavy_count, S.tiles_x * S.tiles_y, eflags, framebuffer, tile_counter};
+    PaintInputs in{segs, recs, tile_range, heavy, heavy_count, S.tiles_x * S.tiles_y, eflags, framebuffer, tile_counter, out.cache_solid_wide};
     // Persistent warps: enough CTAs to fill every SM at the kernel's occupancy (per device).
     // Option paint_wide = 1 selects the build with up to 168 registers (6 CTAs / SM) instead of 128 (8 CTAs / SM).
-    static int blocks_per_sm[2][kMaxDevices] = {{0}};
+    // Every output format has its own instantiation, so the occupancy is kept per format as well.
+    static int blocks_per_sm[3][2][kMaxDevices] = {};
     static std::mutex config_mu;  // several host threads may render on one device
     const int wide = options().paint_wide ? 1 : 0;
+    const uint32_t fmt = out.format <= kFormatRgba32f ? out.format : kFormatRgba8;
+    using Kernel = void (*)(PaintScene, PaintInputs, uint32_t);
+    static const Kernel kernels[3][2] = {{paint_kernel<8, kFormatRgba8>, paint_kernel<6, kFormatRgba8>},
+                                         {paint_kernel<8, kFormatRgba16f>, paint_kernel<6, kFormatRgba16f>},
+                                         {paint_kernel<8, kFormatRgba32f>, paint_kernel<6, kFormatRgba32f>}};
+    const Kernel kernel = kernels[fmt][wide];
     int per_sm = 0;
     {
         std::lock_guard<std::mutex> lk(config_mu);
-        int& slot = blocks_per_sm[wide][current_device_index()];
+        int& slot = blocks_per_sm[fmt][wide][current_device_index()];
         if (!slot) {
-            if (wide) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&slot, paint_kernel<6>, kPaintWarpsPerBlock * 32, 0);
-            else cudaOccupancyMaxActiveBlocksPerMultiprocessor(&slot, paint_kernel<8>, kPaintWarpsPerBlock * 32, 0);
+            cudaOccupancyMaxActiveBlocksPerMultiprocessor(&slot, kernel, kPaintWarpsPerBlock * 32, 0);
             if (slot < 1) slot = 1;
         }
         per_sm = slot;
     }
     const uint32_t want = (uint32_t)(per_sm * device_sm_count());
     const uint32_t need = (n_tiles + kPaintWarpsPerBlock - 1) / kPaintWarpsPerBlock;
-    if (wide) paint_kernel<6><<<min(want, need), kPaintWarpsPerBlock * 32, 0, st>>>(S, in, n_tiles);
-    else paint_kernel<8><<<min(want, need), kPaintWarpsPerBlock * 32, 0, st>>>(S, in, n_tiles);
+    kernel<<<min(want, need), kPaintWarpsPerBlock * 32, 0, st>>>(S, in, n_tiles);
 }
 
 }  // namespace forma

@@ -289,13 +289,15 @@ void Composition::layer_clear(Layer* layer) {  // layer.rs:131-146
 // Renderer
 // ---------------------------------------------------------------------------
 // BufferLayerCache (cpu/buffer/mod.rs:114-197). The per-tile records live on the
-// device (the painter reads and updates them); the host only keeps the size and
-// clear colour of the last frame.
+// device (the painter reads and updates them); the host only keeps the size, output
+// format and clear colour of the last frame.
 struct LayerCache {
     uint8_t id = 0;
-    DeviceBuffer<uint2> tiles;  // CachedTile per tile, see PaintScene::cache_tiles
+    DeviceBuffer<uint2> tiles;       // CachedTile per tile, see PaintScene::cache_tiles
+    DeviceBuffer<uint4> solid_wide;  // float formats: per-tile solid colour at output precision
     bool has_size = false;
     uint64_t width = 0, height = 0;
+    uint32_t format = kFormatRgba8;
     bool has_clear = false;
     float clear_color[4] = {0, 0, 0, 0};
     bool needs_reset = true;  // the tile records must be zeroed before their next use
@@ -467,7 +469,7 @@ class Renderer {
     int rasterize(Composition& comp, uint32_t width, uint32_t height, float band_lo, float band_hi, uint32_t* n_out);
     int render(Composition& comp, uint8_t* buffer, bool buffer_on_device, uint64_t width, uint64_t stride,
                uint64_t height, const uint32_t channels[4], const float clear[4], const forma_rect* crop,
-               LayerCache* cache, forma_timings* timings);
+               LayerCache* cache, forma_timings* timings, uint32_t format = kFormatRgba8);
 };
 
 int Renderer::read_total(uint32_t slot, uint32_t* out) {
@@ -894,11 +896,21 @@ int Renderer::prefetch(Composition& comp, uint64_t width, uint64_t height, const
 
 int Renderer::render(Composition& comp, uint8_t* buffer, bool buffer_on_device, uint64_t width, uint64_t stride,
                      uint64_t height, const uint32_t channels_in[4], const float clear[4], const forma_rect* crop,
-                     LayerCache* cache, forma_timings* timings) {
+                     LayerCache* cache, forma_timings* timings, uint32_t format) {
+    if (format > kFormatRgba32f) {
+        set_error("invalid output format %u", format);
+        return FORMA_STATUS_INVALID;
+    }
+    const uint64_t bpp = format_bytes_per_pixel(format), elem = format_element_bytes(format);
     // LinearLayout::new asserts (layout/mod.rs:188-193) + consts.rs limits.
-    if (!buffer || width == 0 || height == 0 || width * 4 > stride || width > FORMA_MAX_WIDTH || height > FORMA_MAX_HEIGHT) {
+    if (!buffer || width == 0 || height == 0 || width * bpp > stride || width > FORMA_MAX_WIDTH || height > FORMA_MAX_HEIGHT) {
         set_error("invalid render target %llux%llu stride %llu", (unsigned long long)width, (unsigned long long)height,
                   (unsigned long long)stride);
+        return FORMA_STATUS_INVALID;
+    }
+    if (stride % elem != 0 || reinterpret_cast<uintptr_t>(buffer) % elem != 0) {
+        set_error("float frame: stride %llu and buffer address must be multiples of %llu bytes", (unsigned long long)stride,
+                  (unsigned long long)elem);
         return FORMA_STATUS_INVALID;
     }
     FORMA_CUDA_TRY(cudaSetDevice(device));
@@ -922,6 +934,8 @@ int Renderer::render(Composition& comp, uint8_t* buffer, bool buffer_on_device, 
     S.width = (uint32_t)width;
     S.height = (uint32_t)height;
     S.stride = (uint32_t)stride;
+    FrameOut frame_out;
+    frame_out.format = format;
     S.tiles_x = (S.width + 15u) / 16u;
     S.tiles_y = (S.height + 15u) / 16u;
     S.tx_lo = 0; S.tx_hi = S.tiles_x; S.ty_lo = 0; S.ty_hi = S.tiles_y;
@@ -956,10 +970,13 @@ int Renderer::render(Composition& comp, uint8_t* buffer, bool buffer_on_device, 
     const bool pack_written = cache && !buffer_on_device;
     if (cache) {  // renderer.rs:94-110
         const size_t cache_tiles = (size_t)S.tiles_x * S.tiles_y;
-        if (!cache->has_size || cache->width != width || cache->height != height) {
+        // A frame of another output format starts the cache over like a new size does: its
+        // solid colours were compared at another precision.
+        if (!cache->has_size || cache->width != width || cache->height != height || cache->format != format) {
             cache->has_size = true;
             cache->width = width;
             cache->height = height;
+            cache->format = format;
             cache->clear();
         }
         FORMA_CUDA_TRY(cache->tiles.reserve(cache_tiles));
@@ -968,6 +985,10 @@ int Renderer::render(Composition& comp, uint8_t* buffer, bool buffer_on_device, 
             cache->needs_reset = false;
         }
         S.cache_tiles = cache->tiles.ptr;
+        if (format != kFormatRgba8) {  // read only where a tile's has-solid bit is set, i.e. after it was written
+            FORMA_CUDA_TRY(cache->solid_wide.reserve(cache_tiles));
+            frame_out.cache_solid_wide = cache->solid_wide.ptr;
+        }
         S.clear_unchanged = cache->has_clear && cache->clear_color[0] == clear[0] && cache->clear_color[1] == clear[1] &&
                             cache->clear_color[2] == clear[2] && cache->clear_color[3] == clear[3];
         // Layer::is_unchanged(cache_id) per style slot (renderer.rs:144-157); the slots
@@ -1251,16 +1272,16 @@ int Renderer::render(Composition& comp, uint8_t* buffer, bool buffer_on_device, 
             Sb.ty_hi = S.ty_lo + paint_rows * (k + 1u) / kCopyBands;
             cudaStream_t bs = kCopyBands > 1u ? band_stream[k] : stream;
             if (kCopyBands > 1u) FORMA_CUDA_TRY(cudaStreamWaitEvent(bs, band_ev[kMaxCopyBands], 0));
-            launch_paint(Sb, segs.ptr, recs.ptr, tile_range.ptr, heavy_lists, heavy_counts, eflags.ptr, fb, totals.ptr + 16 + k, bs);
+            launch_paint(Sb, segs.ptr, recs.ptr, tile_range.ptr, heavy_lists, heavy_counts, eflags.ptr, fb, totals.ptr + 16 + k, bs, frame_out);
             ++launches;
             const uint64_t y0 = (uint64_t)Sb.ty_lo * 16u, y1 = std::min<uint64_t>((uint64_t)Sb.ty_hi * 16u, height);
             if (x1 > x0 && y1 > y0) {
-                if (x0 == 0 && x1 * 4 == stride)  // whole rows without padding: one contiguous copy
+                if (x0 == 0 && x1 * bpp == stride)  // whole rows without padding: one contiguous copy
                     FORMA_CUDA_TRY(cudaMemcpyAsync(buffer + y0 * stride, fb + y0 * stride, (y1 - y0) * stride, cudaMemcpyDeviceToHost, bs));
                 else
-                    FORMA_CUDA_TRY(cudaMemcpy2DAsync(buffer + y0 * stride + x0 * 4, stride, fb + y0 * stride + x0 * 4, stride,
-                                                     (x1 - x0) * 4, y1 - y0, cudaMemcpyDeviceToHost, bs));
-                d2h_bytes += (x1 - x0) * 4 * (y1 - y0);
+                    FORMA_CUDA_TRY(cudaMemcpy2DAsync(buffer + y0 * stride + x0 * bpp, stride, fb + y0 * stride + x0 * bpp, stride,
+                                                     (x1 - x0) * bpp, y1 - y0, cudaMemcpyDeviceToHost, bs));
+                d2h_bytes += (x1 - x0) * bpp * (y1 - y0);
             }
             if (kCopyBands > 1u) FORMA_CUDA_TRY(cudaEventRecord(band_ev[k], bs));
         }
@@ -1268,7 +1289,7 @@ int Renderer::render(Composition& comp, uint8_t* buffer, bool buffer_on_device, 
         paint_launches = kCopyBands;
         copied_in_bands = true;
     } else {
-        launch_paint(S, segs.ptr, recs.ptr, tile_range.ptr, heavy_lists, heavy_counts, eflags.ptr, fb, totals.ptr + 3, stream);
+        launch_paint(S, segs.ptr, recs.ptr, tile_range.ptr, heavy_lists, heavy_counts, eflags.ptr, fb, totals.ptr + 3, stream, frame_out);
         ++launches;
     }
     FORMA_CUDA_TRY(cudaGetLastError());
@@ -1279,8 +1300,9 @@ int Renderer::render(Composition& comp, uint8_t* buffer, bool buffer_on_device, 
         // With a layer cache only the tiles this frame wrote may touch the host
         // buffer (TileWriteOp::None leaves its bytes alone): pack them on the
         // device, copy count + ids + pixels, scatter on the host.
-        FORMA_CUDA_TRY(packed_tiles.reserve((size_t)S.tiles_x * S.tiles_y * 256u));
-        launch_gather_tiles(S, fb, packed_tiles.ptr, stream);
+        const size_t tile_words = 64u * bpp;  // one packed tile: 256 pixels of bpp bytes, in u32 words
+        FORMA_CUDA_TRY(packed_tiles.reserve((size_t)S.tiles_x * S.tiles_y * tile_words));
+        launch_gather_tiles(S, format, fb, packed_tiles.ptr, stream);
         ++launches;
         uint32_t n_written = 0;
         st = read_total(6, &n_written);
@@ -1288,35 +1310,46 @@ int Renderer::render(Composition& comp, uint8_t* buffer, bool buffer_on_device, 
         last_written_tiles = n_written;
         if (n_written) {
             FORMA_CUDA_TRY(h_written_list.reserve(n_written));
-            FORMA_CUDA_TRY(h_packed_tiles.reserve((size_t)n_written * 256u));
+            FORMA_CUDA_TRY(h_packed_tiles.reserve((size_t)n_written * tile_words));
             FORMA_CUDA_TRY(cudaMemcpyAsync(h_written_list.ptr, written_list.ptr, n_written * sizeof(uint32_t),
                                            cudaMemcpyDeviceToHost, stream));
-            FORMA_CUDA_TRY(cudaMemcpyAsync(h_packed_tiles.ptr, packed_tiles.ptr, (size_t)n_written * 1024u,
+            FORMA_CUDA_TRY(cudaMemcpyAsync(h_packed_tiles.ptr, packed_tiles.ptr, (size_t)n_written * tile_words * 4u,
                                            cudaMemcpyDeviceToHost, stream));
             FORMA_CUDA_TRY(cudaStreamSynchronize(stream));
-            d2h_bytes += (uint64_t)n_written * (1024u + 4u);
-            for (uint32_t i = 0; i < n_written; ++i) {  // LinearLayout::write, layout/mod.rs:265-282
-                const uint32_t tile = h_written_list.ptr[i];
-                const uint64_t x0 = (uint64_t)(tile % S.tiles_x) * 16u, y0 = (uint64_t)(tile / S.tiles_x) * 16u;
-                const uint64_t cols = std::min<uint64_t>(16u, width - x0), rows = std::min<uint64_t>(16u, height - y0);
-                const uint32_t* src = h_packed_tiles.ptr + (size_t)i * 256u;
-                uint8_t* dst = buffer + y0 * stride + x0 * 4u;
-                if (cols == 16u) {  // whole tile rows: fixed-size copies the compiler turns into vector moves
-                    for (uint64_t r = 0; r < rows; ++r) std::memcpy(dst + r * stride, src + r * 16u, 64);
-                } else {
-                    for (uint64_t r = 0; r < rows; ++r) std::memcpy(dst + r * stride, src + r * 16u, cols * 4u);
+            d2h_bytes += (uint64_t)n_written * (tile_words * 4u + 4u);
+            if (format == kFormatRgba8) {
+                for (uint32_t i = 0; i < n_written; ++i) {  // LinearLayout::write, layout/mod.rs:265-282
+                    const uint32_t tile = h_written_list.ptr[i];
+                    const uint64_t x0 = (uint64_t)(tile % S.tiles_x) * 16u, y0 = (uint64_t)(tile / S.tiles_x) * 16u;
+                    const uint64_t cols = std::min<uint64_t>(16u, width - x0), rows = std::min<uint64_t>(16u, height - y0);
+                    const uint32_t* src = h_packed_tiles.ptr + (size_t)i * 256u;
+                    uint8_t* dst = buffer + y0 * stride + x0 * 4u;
+                    if (cols == 16u) {  // whole tile rows: fixed-size copies the compiler turns into vector moves
+                        for (uint64_t r = 0; r < rows; ++r) std::memcpy(dst + r * stride, src + r * 16u, 64);
+                    } else {
+                        for (uint64_t r = 0; r < rows; ++r) std::memcpy(dst + r * stride, src + r * 16u, cols * 4u);
+                    }
+                }
+            } else {
+                for (uint32_t i = 0; i < n_written; ++i) {
+                    const uint32_t tile = h_written_list.ptr[i];
+                    const uint64_t x0 = (uint64_t)(tile % S.tiles_x) * 16u, y0 = (uint64_t)(tile / S.tiles_x) * 16u;
+                    const uint64_t cols = std::min<uint64_t>(16u, width - x0), rows = std::min<uint64_t>(16u, height - y0);
+                    const uint8_t* src = reinterpret_cast<const uint8_t*>(h_packed_tiles.ptr + (size_t)i * tile_words);
+                    uint8_t* dst = buffer + y0 * stride + x0 * bpp;
+                    for (uint64_t r = 0; r < rows; ++r) std::memcpy(dst + r * stride, src + r * 16u * bpp, cols * bpp);
                 }
             }
         }
     } else if (!buffer_on_device && !copied_in_bands) {
         // Only the cropped tile rectangle is written by the reference
-        // (cpu/painter/mod.rs:524-529,589-593); padding bytes beyond width*4 stay untouched.
+        // (cpu/painter/mod.rs:524-529,589-593); padding bytes beyond width*bpp stay untouched.
         uint64_t x0 = (uint64_t)S.tx_lo * 16u, x1 = std::min<uint64_t>((uint64_t)S.tx_hi * 16u, width);
         uint64_t y0 = (uint64_t)S.ty_lo * 16u, y1 = std::min<uint64_t>((uint64_t)S.ty_hi * 16u, height);
         if (x1 > x0 && y1 > y0) {
-            FORMA_CUDA_TRY(cudaMemcpy2DAsync(buffer + y0 * stride + x0 * 4, stride, fb + y0 * stride + x0 * 4, stride,
-                                             (x1 - x0) * 4, y1 - y0, cudaMemcpyDeviceToHost, stream));
-            d2h_bytes += (x1 - x0) * 4 * (y1 - y0);
+            FORMA_CUDA_TRY(cudaMemcpy2DAsync(buffer + y0 * stride + x0 * bpp, stride, fb + y0 * stride + x0 * bpp, stride,
+                                             (x1 - x0) * bpp, y1 - y0, cudaMemcpyDeviceToHost, stream));
+            d2h_bytes += (x1 - x0) * bpp * (y1 - y0);
         }
     }
     FORMA_CUDA_TRY(cudaEventRecord(timer.ev[6], stream));
@@ -1772,6 +1805,27 @@ int forma_renderer_render_device(forma_renderer* r, forma_composition* c, uint8_
                            cache ? &cache->c : nullptr, timings);
     });
 }
+// Float frames are not sliced (sliced_host_render): the slice pipeline is off by default and
+// measured not to pay (DESIGN.md section 3), so it is left as it is for RGBA8.
+int forma_renderer_render_format(forma_renderer* r, forma_composition* c, void* buffer, uint32_t format, uint64_t width,
+                                 uint64_t stride, uint64_t height, const uint32_t channels[4], const float clear[4],
+                                 const forma_rect* crop, forma_layer_cache* cache, forma_timings* timings) {
+    if (format == FORMA_FORMAT_RGBA8)
+        return forma_renderer_render(r, c, static_cast<uint8_t*>(buffer), width, stride, height, channels, clear, crop, cache, timings);
+    return guarded((int)FORMA_ERR_CAPACITY, [&] {
+        return r->r.render(c->c, static_cast<uint8_t*>(buffer), false, width, stride, height, channels, clear, crop,
+                           cache ? &cache->c : nullptr, timings, format);
+    });
+}
+int forma_renderer_render_device_format(forma_renderer* r, forma_composition* c, void* device_buffer, uint32_t format,
+                                        uint64_t width, uint64_t stride, uint64_t height, const uint32_t channels[4],
+                                        const float clear[4], const forma_rect* crop, forma_layer_cache* cache,
+                                        forma_timings* timings) {
+    return guarded((int)FORMA_ERR_CAPACITY, [&] {
+        return r->r.render(c->c, static_cast<uint8_t*>(device_buffer), true, width, stride, height, channels, clear, crop,
+                           cache ? &cache->c : nullptr, timings, format);
+    });
+}
 // --- shared frames (multi-GPU, see include/forma_b200.h) -----------------------
 static_assert(sizeof(cudaIpcMemHandle_t) == sizeof(forma_ipc_handle), "CUDA IPC handles are 64 bytes");
 int forma_shared_frame_create(int device, uint64_t bytes, void** device_ptr, forma_ipc_handle* handle) {
@@ -1907,7 +1961,8 @@ struct forma_renderer_multi {
 
 static int multi_render_impl(forma_renderer_multi* m, forma_composition* c, uint8_t* buffer, bool on_device, uint64_t width,
                              uint64_t stride, uint64_t height, const uint32_t channels[4], const float clear[4],
-                             const forma_rect* crop, forma_timings* timings, size_t n_use = 0, bool chained_uploads = false) {
+                             const forma_rect* crop, forma_timings* timings, uint32_t format = kFormatRgba8, size_t n_use = 0,
+                             bool chained_uploads = false) {
     const size_t n = n_use ? std::min(n_use, m->dev.size()) : m->dev.size();
     m->active = n;
     if (!n || !width || !height || width > FORMA_MAX_WIDTH || height > FORMA_MAX_HEIGHT) {
@@ -1981,7 +2036,7 @@ static int multi_render_impl(forma_renderer_multi* m, forma_composition* c, uint
         if (!band_of(i, &band)) return;
         Renderer& R = m->dev[i]->r;
         status[i] = guarded((int)FORMA_ERR_CAPACITY, [&] {
-            return R.render(comp, buffer, on_device, width, stride, height, channels, clear, &band, nullptr, &tms[i]);
+            return R.render(comp, buffer, on_device, width, stride, height, channels, clear, &band, nullptr, &tms[i], format);
         });
         if (status[i]) {
             errors[i] = forma_last_error();
@@ -2208,7 +2263,7 @@ static int sliced_host_render(forma_renderer* r, forma_composition* c, uint8_t* 
         FORMA_CUDA_TRY(cudaStreamWaitEvent(Q.stream, P.count_ev, 0));
         before[i] = {Q.launches, Q.h2d_bytes, Q.d2h_bytes};
     }
-    const int st = multi_render_impl(m, c, buffer, false, width, stride, height, channels, clear, crop, timings, n,
+    const int st = multi_render_impl(m, c, buffer, false, width, stride, height, channels, clear, crop, timings, kFormatRgba8, n,
                                      options().slice_chain != 0);
     if (st) return st;
     // What the caller reads from this renderer after a frame: sums over the slices; stage times:
@@ -2271,6 +2326,23 @@ int forma_renderer_multi_render_device(forma_renderer_multi* m, forma_compositio
                                        const float clear[4], const forma_rect* crop, forma_timings* timings) {
     return guarded((int)FORMA_ERR_CAPACITY, [&] {
         return multi_render_impl(m, c, buffer_on_first_device, true, width, stride, height, channels, clear, crop, timings);
+    });
+}
+int forma_renderer_multi_render_format(forma_renderer_multi* m, forma_composition* c, void* buffer, uint32_t format, uint64_t width,
+                                       uint64_t stride, uint64_t height, const uint32_t channels[4], const float clear[4],
+                                       const forma_rect* crop, forma_timings* timings) {
+    return guarded((int)FORMA_ERR_CAPACITY, [&] {
+        return multi_render_impl(m, c, static_cast<uint8_t*>(buffer), false, width, stride, height, channels, clear, crop, timings,
+                                 format);
+    });
+}
+int forma_renderer_multi_render_device_format(forma_renderer_multi* m, forma_composition* c, void* buffer_on_first_device,
+                                              uint32_t format, uint64_t width, uint64_t stride, uint64_t height,
+                                              const uint32_t channels[4], const float clear[4], const forma_rect* crop,
+                                              forma_timings* timings) {
+    return guarded((int)FORMA_ERR_CAPACITY, [&] {
+        return multi_render_impl(m, c, static_cast<uint8_t*>(buffer_on_first_device), true, width, stride, height, channels, clear,
+                                 crop, timings, format);
     });
 }
 /* Tile-row boundaries of the bands the next frame will use (n + 1 values) and the

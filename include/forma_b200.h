@@ -204,6 +204,33 @@ int forma_renderer_render_device(forma_renderer*, forma_composition*, uint8_t* d
                                  const forma_rect* crop, forma_layer_cache* cache,
                                  forma_timings* timings);
 
+/* Output formats of a frame (the *_format calls below; the calls without the suffix are RGBA8).
+ *  - RGBA8: sRGB-encoded bytes, what cpu::Renderer writes (compute_srgb, cpu/painter/mod.rs:466-483).
+ *  - RGBA32F: per pixel the four f32 values compute_srgb would receive, before any encode: the
+ *    painter's linear accumulator as is (not clamped, not (un)premultiplied; alpha linear as in
+ *    RGBA8), 16 bytes. A tile the optimiser folds to one solid colour holds that colour (the value
+ *    to_srgb_bytes receives, mod.rs:692).
+ *  - RGBA16F: the same values as IEEE binary16, round to nearest even (overflow -> +-inf, NaN stays
+ *    NaN), 8 bytes: the format of the reference's gpu::Renderer texture (Rgba16Float).
+ * Channel order follows `channels` exactly as for bytes (Zero -> 0.0, One -> 1.0, Alpha -> One when
+ * clear_color.a == 1). Layout (width_stride in BYTES), crops, partial edge tiles and layer-cache
+ * damage follow the RGBA8 rules. A layer cache compares a solid tile's colour with last frame's at
+ * the output precision (the halves / the f32 bit patterns), and a frame of another format than the
+ * cache's last one starts the cache over, like a new size does.
+ * FORMA_ERR_INVALID_ARGUMENT: unknown format, width * bytes_per_pixel > width_stride, or a stride
+ * or buffer address that is not a multiple of the element size (2 bytes RGBA16F, 4 bytes RGBA32F). */
+enum { FORMA_FORMAT_RGBA8 = 0, FORMA_FORMAT_RGBA16F = 1, FORMA_FORMAT_RGBA32F = 2 };
+int forma_renderer_render_format(forma_renderer*, forma_composition*, void* buffer, uint32_t format, uint64_t width,
+                                 uint64_t width_stride, uint64_t height, const uint32_t channels[4],
+                                 const float clear_color[4], const forma_rect* crop, forma_layer_cache* cache,
+                                 forma_timings* timings);
+/* The frame stays in HBM: with RGBA16F it is what gpu::Renderer::render_to_texture leaves in its
+ * texture, ready for a consumer on the same device (e.g. a torch tensor's data_ptr()). */
+int forma_renderer_render_device_format(forma_renderer*, forma_composition*, void* device_buffer, uint32_t format,
+                                        uint64_t width, uint64_t width_stride, uint64_t height,
+                                        const uint32_t channels[4], const float clear_color[4],
+                                        const forma_rect* crop, forma_layer_cache* cache, forma_timings* timings);
+
 /* Launch on `cuda_stream` (a cudaStream_t, e.g. torch.cuda.current_stream().cuda_stream)
  * instead of the default stream. */
 void forma_renderer_set_stream(forma_renderer*, void* cuda_stream);
@@ -226,6 +253,16 @@ int forma_renderer_multi_render_device(forma_renderer_multi*, forma_composition*
                                        uint64_t width, uint64_t width_stride, uint64_t height,
                                        const uint32_t channels[4], const float clear_color[4],
                                        const forma_rect* crop, forma_timings* timings);
+/* The same in any FORMA_FORMAT_* (see forma_renderer_render_format): every device's band lands in
+ * the host buffer / the first device's frame at the format's width. */
+int forma_renderer_multi_render_format(forma_renderer_multi*, forma_composition*, void* buffer, uint32_t format,
+                                       uint64_t width, uint64_t width_stride, uint64_t height,
+                                       const uint32_t channels[4], const float clear_color[4],
+                                       const forma_rect* crop, forma_timings* timings);
+int forma_renderer_multi_render_device_format(forma_renderer_multi*, forma_composition*, void* buffer_on_first_device,
+                                              uint32_t format, uint64_t width, uint64_t width_stride, uint64_t height,
+                                              const uint32_t channels[4], const float clear_color[4],
+                                              const forma_rect* crop, forma_timings* timings);
 /* bounds[n + 1]: tile-row boundaries of the bands the next frame will use; band_ms[n]:
  * device-timeline ms of every band in the last frame. Returns n. */
 int forma_renderer_multi_bands(const forma_renderer_multi*, uint32_t* bounds, double* band_ms);
